@@ -20,6 +20,11 @@ value = N x (iterations / s): 500k-class-shard iterations per second.
 
 --impl reference : the CPU path (oracle port, OpenMP over all host cores) on the same
 workload; each step is a bounded sample of iterations.
+
+--dump-outputs DIR : after the timed steps, what the last timed step of each path returned to its caller, as
+DIR/<name>.npy in float64 (see collect_outputs); the inputs are seeded, so two builds can be compared array by array.
+
+The bench writes nothing into the source tree (it may be read-only): what it compiles or caches goes to temp dirs.
 """
 import argparse
 import json
@@ -27,11 +32,13 @@ import os
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True
 
 
 def _bind_rank_to_cores():
@@ -171,8 +178,17 @@ class ClockSampler:
 
 
 _CPU_BEST = {}
-CPU_PROBE_FILE = os.path.join(ROOT, ".cpu_probe.json")     # git-ignored; per box (it does not travel back)
+CPU_PROBE_FILE = os.path.join(tempfile.gettempdir(), f"salmon_b200_cpu_probe_{os.getuid()}.json")     # per box and user
 CPU_REPEATS = 5
+_SCRATCH = None
+
+
+def scratch_dir():
+    """a temporary directory for this run (removed at exit): host helpers the bench compiles go there"""
+    global _SCRATCH
+    if _SCRATCH is None:
+        _SCRATCH = tempfile.TemporaryDirectory(prefix="sb_bench_")
+    return _SCRATCH.name
 
 
 def _cpu_probe_load():
@@ -191,8 +207,8 @@ def cpu_port_rate(eq, proj, eff, uniq, vbem, budget_s, threads):
     The port mirrors the reference's decomposition (parallel_for over classes + CAS f64 adds).  On many-core
     hosts that decomposition is contention-bound, so the thread count is chosen ONCE per box by a probe over
     {all, 64, 32, 16, 8} cores and the serial restatement (median of three differences per candidate); the
-    choice is written to .cpu_probe.json and reused by every later call on that box (the driver runs the
-    reference arm and then this arm on the same box: both time the same thread count).  Threads are pinned
+    choice is written to CPU_PROBE_FILE and reused by every later call on that box (a reference-arm run and a
+    B200-arm run on the same box time the same thread count).  Threads are pinned
     (OMP_PROC_BIND=close, OMP_PLACES=cores, set before libgomp loads).  The reported rate is the MEDIAN of
     CPU_REPEATS timed runs; returns (rate, iterations per run, threads, [rates])."""
     import oracle_lib as O
@@ -336,7 +352,7 @@ def stage_a_from_gz(idx, d, f1, f2, n, L, batch, threads, max_pairs=1_000_000):
             raise RuntimeError("gzip failed")
     out = {"files": "the first %d pairs, gzip -1" % k, "pairs": int(k), "parser_threads": threads,
            "gz_bytes": int(sum(os.path.getsize(g) for g in gz))}
-    r = subprocess.run([sys.executable, "-c", _GZ_PARSER_SNIPPET, ROOT, gz[0], gz[1], str(batch), str(L), str(threads), str(k)],
+    r = subprocess.run([sys.executable, "-B", "-c", _GZ_PARSER_SNIPPET, ROOT, gz[0], gz[1], str(batch), str(L), str(threads), str(k)],
                        capture_output=True, text=True, timeout=180)
     m = re.search(r"PARSER_RATE ([0-9.eE+-]+)", r.stdout)
     if r.returncode != 0 or not m:
@@ -424,6 +440,7 @@ def stage_a_from_files(idx, left, right, batch, ncores):
 def stage_a_cpu(idx, p, left, right, budget_s, ncores):
     """CPU port (the product's serial forms compiled for the host, OpenMP over reads) on a bounded sample."""
     import hostmap_lib
+    hostmap_lib.SO = os.path.join(scratch_dir(), "libhostmap.so")
     probe = min(20_000, left.shape[0])
     dt, _, _ = hostmap_lib.map_throughput(idx, p, left[:probe], right[:probe], 0, ncores)
     n = int(min(left.shape[0], max(probe, probe * budget_s / max(dt, 1e-3))))
@@ -504,7 +521,7 @@ def bench_stage_a(args, rank, world, local, dist, W, peak, peak_src, ncores):
     res_t = reduce_max(statistics.mean(res_s)); e2e_t = reduce_max(statistics.mean(e2e_s))
     if rank != 0:
         ctx.close()
-        return None
+        return None, None
     d2h = sum(res[k].nbytes for k in ("off", "tids", "weights", "counts", "projected_counts", "eff_len", "unique_counts",
                                      "total_counts")) + (res["bins"].nbytes if res["bins"] is not None else 0)
     seed_launch_ms = statistics.mean(seed_ms_l) / max(seed_n_l, 1)
@@ -555,7 +572,57 @@ def bench_stage_a(args, rank, world, local, dist, W, peak, peak_src, ncores):
             out["from_files"] = stage_a_from_files(idx, left, right, batch, ncores)
     if ctx is not None:
         ctx.close()
+    return out, res
+
+
+DUMP_BYTES = 64 << 20
+
+
+def class_order(res):
+    """the classes of an sb_map_finish result sorted by label (transcripts, then range-factorisation bins): the device
+    emits them in hash-table order, which differs from run to run"""
+    off = res["off"].astype(np.int64).tolist()
+    tids = res["tids"].tolist()
+    bins = res["bins"].tolist() if res["bins"] is not None else None
+    labels = [tids[a:b] + (bins[a:b] if bins is not None else []) for a, b in zip(off[:-1], off[1:])]
+    return np.array(sorted(range(len(labels)), key=labels.__getitem__), dtype=np.int64)
+
+
+def collect_outputs(alpha, alpha_e2e, stage_a_res):
+    """What the last timed step of each path handed to its caller, by name:
+      em_alpha, em_alpha_e2e  the abundances from sb_em_run (class table resident) and from sb_em_optimize (host buffers)
+      stage_a_<name>          the per-transcript EM inputs from sb_map_finish
+      stage_a_class_<name>    its class table in label order: per class sizes and counts, per entry tids, weights, bins;
+                              a seeded sample of the classes if all of them would take the output past DUMP_BYTES"""
+    out = {"em_alpha": alpha, "em_alpha_e2e": alpha_e2e}
+    if stage_a_res is None:
+        return out
+    r = stage_a_res
+    for k in ("projected_counts", "eff_len", "unique_counts", "total_counts"):
+        out["stage_a_" + k] = r[k]
+    off = r["off"].astype(np.int64)
+    sizes = np.diff(off)
+    fields = ("tids", "weights") + (("bins",) if r["bins"] is not None else ())
+    order = class_order(r)
+    room = DUMP_BYTES // 8 - 1024 - sum(a.size for a in out.values())      # float64 values left (1024: the .npy headers)
+    cost = 2 + len(fields) * sizes[order]
+    if cost.sum() > room:
+        perm = np.random.default_rng(0).permutation(len(order))
+        order = order[np.sort(perm[:np.searchsorted(np.cumsum(cost[perm]), room, side="right")])]
+    sz = sizes[order]
+    entries = np.repeat(off[:-1][order] - np.concatenate(([0], np.cumsum(sz)[:-1])), sz) + np.arange(sz.sum())
+    out["stage_a_class_sizes"] = sz
+    out["stage_a_class_counts"] = r["counts"][order]
+    for k in fields:
+        out["stage_a_class_" + k] = r[k][entries]
     return out
+
+
+def dump_outputs(d, arrays):
+    """every array as d/<name>.npy in float64 (integers below 2**53 are exact in it)"""
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def main():
@@ -570,7 +637,12 @@ def main():
     ap.add_argument("--no-stage-a", action="store_true", help="skip the Stage A (mapping) measurement")
     ap.add_argument("--sa-small", action="store_true", help="Stage A on a 20x smaller transcriptome (dev)")
     ap.add_argument("--no-files", action="store_true", help="skip the FASTQ-files -> classes measurement (row f1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs dumps the B200 arm's outputs")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -610,7 +682,7 @@ def main():
             "cpu_baseline": {"value": val, "unit": "iters/s", "cores": used, "kind": "port", "host_cores": ncores,
                              "sample": f"median over steps; each step = median of {CPU_REPEATS} runs of {sample_iters} "
                                        f"iterations of the same workload; thread count probed once per box "
-                                       f"(best of all/64/32/16/8/serial, cached in .cpu_probe.json), threads pinned"},
+                                       f"(best of all/64/32/16/8/serial, cached in a temp file), threads pinned"},
             "e2e": {"value": val, "unit": "iters/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "gpu_launches": 0,
         }
@@ -733,9 +805,9 @@ def main():
 
     peak, peak_src = measured_peak()
     ctx.close()
-    stage_a = None
+    stage_a, stage_a_res = None, None
     if not args.no_stage_a:
-        stage_a = bench_stage_a(args, rank, world, local, dist, W, peak, peak_src, ncores)
+        stage_a, stage_a_res = bench_stage_a(args, rank, world, local, dist, W, peak, peak_src, ncores)
     if rank != 0:
         if dist is not None:
             dist.destroy_process_group()
@@ -785,11 +857,13 @@ def main():
         line["cpu_baseline"] = {"value": cpu_val, "unit": "iters/s", "cores": cpu_used, "kind": "port",
                                 "host_cores": ncores,
                                 "sample": f"median of {CPU_REPEATS} runs of {cpu_n} iterations of the same workload; thread "
-                                          f"count probed once per box (cached in .cpu_probe.json, shared with the "
+                                          f"count probed once per box (cached in a temp file, shared with the "
                                           f"reference arm), threads pinned",
                                 "runs": [round(x, 1) for x in cpu_rates]}
     if stage_a is not None:
         line["stage_a"] = stage_a
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, collect_outputs(alpha, a2, stage_a_res))
     print(json.dumps(line))
     if dist is not None:
         dist.destroy_process_group()

@@ -92,21 +92,11 @@ def test_product_host_logic_vs_libm_oracle():
 
 def test_oracle_digamma_vs_reference_tree_eigen():
     """the oracle's digamma (checker of the fused VBEM transform) against the digamma the reference tree itself vendors
-    (Eigen's Cephes-derived implementation, compiled by oracle/build_ref.sh from the headers under /root/reference through
-    a five-line shim; boost::math::digamma, which salmon calls, is not in the tree).  Skipped when oracle/_ref is absent."""
-    import ctypes as C
+    (Eigen's Cephes-derived implementation; boost::math::digamma, which salmon calls, is not in the tree), at a seeded
+    sample of arguments stored with Eigen's values in tests/golden/eigen_digamma.npz by tests/golden/make_ref_golden.py"""
     import os
-    import numpy as np
-    import pytest
-    import oracle_lib as O
-    so = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "libeigen_digamma_ref.so")
-    if not os.path.exists(so):
-        pytest.skip("oracle/_ref/libeigen_digamma_ref.so not built (needs /root/reference)")
-    lib = C.CDLL(so)
-    rng = np.random.default_rng(11)
-    x = np.concatenate([10.0 ** rng.uniform(-10, 9, 40000), np.linspace(0.01, 40.0, 20000), rng.uniform(1.3, 1.6, 5000)])
-    ref = np.empty_like(x)
-    lib.ref_eigen_digamma(C.c_ulong(len(x)), x.ctypes.data_as(C.c_void_p), ref.ctypes.data_as(C.c_void_p))
+    g = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "eigen_digamma.npz"))
+    x, ref = g["x"], g["digamma"]
     mine = np.array([O.digamma(v) for v in x])
     err = np.abs(mine - ref)
     # relative where digamma is not near its root (x0 = 1.4616...), absolute there
